@@ -32,6 +32,10 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 N1 = 3162  # interior grid edge: (nx-2) with nx = 3164 (SURVEY 8: L5)
+# --dump-outputs: y has 10M fp64 rows per GPU (80 MB), so a fixed, seeded sample of 2^22 rows over all ranks is written
+# (32 MB); the same arguments give the same rows, so two builds can be compared output for output
+DUMP_ROWS = 1 << 22
+DUMP_SEED = 20240
 METRIC = "csr_spmv_gflops"
 WORKLOAD = "5-pt Laplacian (examples/pde.py operator) 3162x3162 interior grid per GPU, fp64 CSR SpMV, int32 indices"
 
@@ -314,6 +318,11 @@ def run_gpu(args):
     t_end.record()
     barrier()
     clocks = sampler.stop()
+    dump = {}
+    if args.dump_outputs:   # y of the last timed step, as the caller of the product receives it
+        k = min(hi - lo, DUMP_ROWS // world)
+        rows = np.sort(np.random.default_rng(DUMP_SEED + rank).choice(hi - lo, size=k, replace=False))
+        dump["y" if world == 1 else f"y_rank{rank}"] = y[torch.from_numpy(rows).to(y.device)].cpu().numpy()
     elapsed_ms = t_start.elapsed_time(t_end)
     kern_ms = float(np.mean([s.elapsed_time(e) for s, e in kern_ev]))
     bare_ms = kern_ms
@@ -381,6 +390,11 @@ def run_gpu(args):
         else:
             del local
             extras = sharded_rows_of_the_path(torch, dist, bd, gallery, peak, rank, world, args)
+
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
 
     if rank != 0:
         return 0
@@ -793,7 +807,14 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU-baseline sampling (rank 0, N=1)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the CG / SpGEMM side measurements at N=1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write y of the last step (a fixed, seeded sample of its rows, float64) "
+                         "to DIR/y.npy (DIR/y_rank<r>.npy per rank at N>1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU product; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)

@@ -8,9 +8,11 @@ GPU minutes are spent on it; it says nothing about the kernels.
 import os
 import sys
 
-import numpy as np
-import pytest
-import torch
+os.environ["CUDA_VISIBLE_DEVICES"] = ""   # a host run by design: where a GPU is visible, keep the package off it
+
+import numpy as np  # noqa: E402
+import pytest  # noqa: E402
+import torch  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)

@@ -79,6 +79,9 @@ def _patch_ops_with_oracle():
 
 
 def _worker(rank, world, port, case, q):
+    # host process by design (gloo, oracle leaf ops): where GPUs are visible, init_process_group would bind each rank
+    # to GPU `rank` and the package would place shards on it, so hide them before anything initialises CUDA
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""
     try:
         sys.path.insert(0, ROOT)
         sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -294,9 +297,16 @@ def _run(world, case):
     procs = [ctx.Process(target=_worker, args=(r, world, port, case, q)) for r in range(world)]
     for p in procs:
         p.start()
-    results = [q.get(timeout=240) for _ in procs]
-    for p in procs:
-        p.join(timeout=60)
+    results = []
+    try:
+        while len(results) < world and not (results and "error" in results[-1][1]):
+            results.append(q.get(timeout=240))
+    finally:
+        for p in procs:   # after a failure the other ranks wait in a collective: do not leave them running
+            p.join(timeout=60 if len(results) == world else 0)
+            if p.is_alive():
+                p.kill()
+                p.join()
     for rank, out in results:
         assert "error" not in out, f"rank {rank}: {out.get('error')}"
         assert out.get("ok")

@@ -17,6 +17,14 @@ import legate.sparse_b200 as sparse
 from legate.sparse_b200 import _lib
 
 
+@pytest.fixture(autouse=True)
+def _host_tensors(monkeypatch):
+    """Host-side checks: keep the package on host tensors where a GPU is visible too (it would place them there)."""
+    from legate.sparse_b200.runtime import Runtime
+
+    monkeypatch.setattr(Runtime, "has_cuda", property(lambda self: False))
+
+
 def _declared_symbols():
     text = open(os.path.join(ROOT, "include", "b200sparse.h")).read()
     text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)

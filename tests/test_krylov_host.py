@@ -26,6 +26,7 @@ def cpu_ops(monkeypatch, oracle):
     monkeypatch.setattr(_ops, "dot", dot)
     monkeypatch.setattr(_ops, "nrm2", nrm2)
     monkeypatch.setattr(runtime, "require_cuda", lambda what: None)
+    monkeypatch.setattr(type(runtime), "has_cuda", property(lambda self: False))   # host tensors where a GPU is visible too
     return oracle
 
 
